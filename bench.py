@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- PageRank edges/s on synthetic RMAT (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one complete hot-path pass: ParallelIterativePageRank semantics with
 (max_iterations=20, damping=0.85, stop_epsilon=0.0) over the device-resident graph, i.e. 20 power
@@ -31,6 +31,7 @@ import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 ITERATIONS = 20
 DAMPING = 0.85
@@ -44,6 +45,23 @@ HBM_FALLBACK_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+DUMP_SAMPLE = 1 << 21  # elements kept of an output larger than DUMP_SAMPLE * 16 B (32 MiB)
+
+
+def dump_output(directory, name, values):
+    """--dump-outputs: writes what the last timed step returned as DIR/<name>.npy in float64, so that two builds run
+    with the same arguments (same seeded inputs) can be compared output for output.  An output larger than 32 MiB is
+    reduced to a fixed, seeded sample of DUMP_SAMPLE elements, whose positions go to DIR/<name>_index.npy (float64)."""
+    os.makedirs(directory, exist_ok=True)
+    values = np.asarray(values, dtype=np.float64)
+    if values.nbytes > 16 * DUMP_SAMPLE:
+        index = np.sort(np.random.default_rng(SEED).choice(len(values), DUMP_SAMPLE, replace=False))
+        np.save(os.path.join(directory, name + "_index.npy"), index.astype(np.float64))
+        values = values[index]
+    np.save(os.path.join(directory, name + ".npy"), values)
+    log(f"dumped {name} ({len(values)} values) to {directory}")
 
 
 # ---- clocks sampling (nvidia-smi during the timed region) ---------------------------------------------
@@ -428,6 +446,11 @@ def run_b200_arm(args):
         class_ms += np.array(st.class_ms)
         iters = st.iterations
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:  # single GPU (checked in main): d_out holds the ranks of the last timed step
+        ranks = np.empty(n, dtype=np.float64)
+        _check(lib.mgb200_copy_to_host(device, ranks.ctypes.data, d_out, 8 * n))
+        dump_output(args.dump_outputs, "ranks", ranks)
+        del ranks
     total_ms = float(sum(step_ms))
     if dist is not None:
         import torch
@@ -633,6 +656,8 @@ def run_bfs_arm(args):
         level_counts.append(st["levels"])
         launches += st["kernel_launches"]
     e2e_dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "distances", dist)
     total = float(sum(ms))
     # Roofline (HBM-bound integer work).  Algorithmic bytes of one direction-optimising traversal (DESIGN.md 7):
     #   4 B per inspected adjacency entry + 12 B per reached vertex (8 B row offsets, 4 B distance written)
@@ -706,6 +731,8 @@ def run_katz_arm(args):
         cent, st = K.set_katz(g, alpha, eps)
         ms.append(st["iterate_ms"]); iters = st["iterations"]; launches += st["kernel_launches"]
     e2e_dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "centrality", cent)
     total = float(sum(ms))
     info = g.info
     g.close()
@@ -770,7 +797,14 @@ def main():
     ap.add_argument("--workload", default="pagerank", choices=["pagerank", "bfs", "katz"],
                     help="pagerank (the BASELINE metric, default), bfs (config #5) or katz (SURVEY 8f-1)")
     ap.add_argument("--quick", action="store_true", help="sweep mode: device-resident timing only, compact JSON")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output of the last one as DIR/<name>.npy (float64; a fixed "
+                         "seeded sample of outputs over 32 MiB); single-GPU B200 path only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "b200"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl b200")
     global REAL_STDOUT
     sys.stdout.flush()
     REAL_STDOUT = os.dup(1)

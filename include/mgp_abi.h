@@ -4,9 +4,9 @@
  * Written from scratch as DECLARATIONS ONLY: the authoritative definition is the reference's
  * include/mg_procedure.h (2170 lines; memgraph/memgraph @ 292f896a).  Every prototype below names
  * the line of that header it restates, so a maintainer can diff them; the module also compiles
- * against the reference header itself (-DMGB200_USE_REFERENCE_MGP_HEADER -I<reference>/include,
- * exercised by tests/test_module_host.py::test_module_compiles_against_the_reference_header where the checkout exists), which proves the two agree
- * on every call the module makes.
+ * against the reference header itself (-DMGB200_USE_REFERENCE_MGP_HEADER -I<reference>/include),
+ * and tests/test_module_host.py::test_mgp_abi_matches_the_reference_header checks every prototype,
+ * enumerator and layout below against what the reference header gives (recorded under tests/golden/).
  *
  * Exports the module must provide (mg_procedure.h:1780-1793, loader: src/query/procedure/module.cpp:868-929):
  *     int mgp_init_module(struct mgp_module *, struct mgp_memory *);   required, 0 = success

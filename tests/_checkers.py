@@ -1,6 +1,6 @@
-"""ctypes front-ends for the CHECKERS (oracle/): the plain-C restatement and, when it was built
-from /root/reference, the reference's own algorithm.  Only tests/, __graft_entry__.smoke() and
-bench.py's cpu_baseline / --impl reference legs may import this."""
+"""ctypes front-ends for the CHECKERS (oracle/): the plain-C restatement and, when oracle/Makefile
+built it from a reference checkout, the reference's own algorithm.  Only tests/, tests/golden/,
+__graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this."""
 import ctypes
 import os
 import subprocess
@@ -51,6 +51,13 @@ def oracle_rmat_edges(scale, count=None, seed=42, a=0.57, b=0.19, c=0.19, first=
 
 def _u64(a):
     return np.ascontiguousarray(np.asarray(a, dtype=np.uint64))
+
+
+def sha256_of(a, dtype=np.float64):
+    """Hex SHA-256 of the array's little-endian bytes: how golden files store vectors too large to keep whole while
+    still pinning them bit for bit."""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a, dtype=np.dtype(dtype).newbyteorder("<")).tobytes()).hexdigest()
 
 
 class Oracle:

@@ -12,6 +12,11 @@ JSON files.  Sources:
 * ``pagerank_ref_outputs.json``   <- outputs of the reference algorithm itself (oracle/_ref,
   built by oracle/Makefile) on small seeded graphs at several argument settings, 17 digits,
   so the GPU box -- which has no /root/reference -- can still compare against the real thing.
+* ``pagerank_ref_threads.json``, ``katz_ref_outputs.json``, ``pagerank_reference_module.json``,
+  ``mgp_abi_reference.json``      <- what the reference's own binaries under oracle/_ref and its
+  include/mg_procedure.h give on the inputs the tests generate, so a checkout without them still
+  compares against the reference.  Vectors too large to keep whole are stored as the SHA-256 of
+  their little-endian bytes, which keeps the comparisons bit-exact.
 """
 import ctypes
 import json
@@ -133,11 +138,112 @@ def bfs_unit_graph():
     return {"source": "tests/unit/bfs_common.hpp:42-110,423-470", "n": n, "edges": edges, "cases": cases}
 
 
+TESTS = os.path.dirname(HERE)
+
+
+def ref_threads():
+    """The reference algorithm (oracle/_ref/libpagerank_ref.so) on test_oracle.thread_cases, as float64 digests."""
+    sys.path.insert(0, TESTS)
+    from _checkers import OracleError, Reference, sha256_of
+    from test_oracle import THREAD_COUNTS, thread_cases
+    ref = Reference()
+    cases = [{"threads": threads, "n": n, "m": m, "args": kw,
+              "sha256": sha256_of(ref.pagerank(n, frm, to, num_of_threads=threads, **kw))}
+             for threads in THREAD_COUNTS for n, m, frm, to, kw in thread_cases(threads)]
+    try:
+        ref.pagerank(2, [0], [1], num_of_threads=0)
+        raise AssertionError("the reference accepted num_of_threads = 0")
+    except OracleError as ex:
+        zero_threads_error = str(ex)
+    nan = bool(np.all(np.isnan(ref.pagerank(3, [0, 1], [1, 2], damping_factor=1.0, max_iterations=50))))
+    return {"source": "oracle/_ref/libpagerank_ref.so = reference algorithm/pagerank.cpp compiled in place; ranks as "
+                      "SHA-256 of their little-endian float64 bytes",
+            "cases": cases, "edge_cases": {"zero_threads_error": zero_threads_error, "damping_1_all_nan": nan}}
+
+
+def katz_ref():
+    """The reference's katz.cpp (oracle/_ref/libkatz_ref.so) on test_katz_oracle.katz_cases that separate within the
+    oracle's guard (the reference would spin on the others), as float64 digests."""
+    sys.path.insert(0, TESTS)
+    from _checkers import sha256_of
+    from test_katz_oracle import katz_cases, oracle_katz, ref_katz
+    cases = []
+    for n, m, f, t, alpha, eps in katz_cases():
+        if oracle_katz(n, f, t, alpha, eps, guard=2000)[0] == 0:
+            cases.append({"n": n, "m": m, "alpha": alpha, "eps": eps, "sha256": sha256_of(ref_katz(n, f, t, alpha, eps))})
+    return {"source": "oracle/_ref/libkatz_ref.so = reference katz_centrality_module/algorithm/katz.cpp compiled in "
+                      "place; centralities as SHA-256 of their little-endian float64 bytes", "cases": cases}
+
+
+def reference_module():
+    """The reference's pagerank.so (oracle/_ref/pagerank_reference.so) loaded and called through the fake mgp host
+    on the inputs of test_module_host.py and test_gpu_module.py."""
+    import subprocess
+    sys.path.insert(0, TESTS)
+    import _fakehost as fh
+    from _checkers import sha256_of
+    from test_module_host import e2e_fixture_graph, e2e_fixture_rows, scattered_graph
+    out = {"source": "oracle/_ref/pagerank_reference.so = reference mage/cpp/pagerank_module compiled in place, "
+                     "called through tests/mgp_fake_host.cpp; large outputs as SHA-256 of their little-endian bytes"}
+    und = subprocess.run(["nm", "-D", "--undefined-only", fh.REF_MODULE_SO], capture_output=True, text=True,
+                         check=True).stdout
+    out["imports"] = sorted(line.split()[-1] for line in und.splitlines() if " U mgp_" in line)
+    with fh.Module(fh.REF_MODULE_SO) as module:
+        out["signature"] = module.signature()
+        with fh.Graph([1, 2], [1], [2]) as g:
+            try:
+                module.call(g, 10, 0.85, 1e-5, 0)
+                raise AssertionError("the reference module accepted num_of_threads = 0")
+            except fh.ProcedureError as ex:
+                out["zero_threads_error"] = str(ex)
+
+        def digests(graph, args_list):
+            gids, src, dst = graph
+            rows = []
+            with fh.Graph(gids, src, dst) as g:
+                for args in args_list:
+                    nodes, ranks = module.call(g, *args)
+                    rows.append({"args": list(args), "nodes_sha256": sha256_of(nodes, np.int64),
+                                 "ranks_sha256": sha256_of(ranks)})
+            return rows
+
+        out["config1"] = digests(scattered_graph(10_000, 50_000, seed=42), [(), (20, 0.85, 0.0, 8)])
+        out["same_rows"] = digests(scattered_graph(3000, 20000, seed=7), [(), (20, 0.85, 0.0, 4), (7, 0.3, 0.0, 1)])
+        out["e2e"] = {}
+        for case in e2e_cases()["cases"]:
+            gid_of, gids, src, dst = e2e_fixture_graph(case)
+            with fh.Graph(gids, src, dst) as g:
+                out["e2e"][case["name"]] = e2e_fixture_rows(gid_of, *module.call(g, *case["call_args"]))
+        out["unit_vectors"] = []
+        for i, case in enumerate(unit_vectors()["cases"]):
+            if case["m"] != len(case["edges"]):
+                continue
+            gids = np.arange(case["n"], dtype=np.int64) * 5 + 11
+            e = np.array(case["edges"], dtype=np.int64).reshape(-1, 2)
+            with fh.Graph(gids, gids[e[:, 0]] if len(e) else [], gids[e[:, 1]] if len(e) else []) as g:
+                nodes, ranks = module.call(g)
+            out["unit_vectors"].append({"case": i, "nodes": nodes.tolist(), "ranks": ranks.tolist()})
+    return out
+
+
+def mgp_abi_reference():
+    """test_module_host.mgp_abi_probe through the reference's include/mg_procedure.h."""
+    import tempfile
+    sys.path.insert(0, TESTS)
+    from test_module_host import mgp_abi_probe
+    with tempfile.TemporaryDirectory() as tmp:
+        probe = mgp_abi_probe("mg_procedure.h", os.path.join(REF, "include"), tmp)
+    return {"source": "include/mg_procedure.h: typeid(function).name() of every function include/mgp_abi.h declares, "
+                      "the value of every enumerator it declares, and the layout of mgp_vertex_id", "probe": probe}
+
+
 def main():
     if not os.path.isdir(REF):
         sys.exit("reference checkout not present; golden fixtures are committed, nothing to do")
     for name, fn in [("pagerank_unit_vectors.json", unit_vectors), ("pagerank_e2e_cases.json", e2e_cases),
-                     ("pagerank_ref_outputs.json", ref_outputs), ("bfs_unit_graph.json", bfs_unit_graph)]:
+                     ("pagerank_ref_outputs.json", ref_outputs), ("bfs_unit_graph.json", bfs_unit_graph),
+                     ("pagerank_ref_threads.json", ref_threads), ("katz_ref_outputs.json", katz_ref),
+                     ("pagerank_reference_module.json", reference_module), ("mgp_abi_reference.json", mgp_abi_reference)]:
         with open(os.path.join(HERE, name), "w") as f:
             json.dump(fn(), f, indent=None if "ref_outputs" in name else 1, separators=(",", ":") if "ref_outputs" in name else None)
             f.write("\n")

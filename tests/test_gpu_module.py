@@ -1,6 +1,6 @@
 """-m gpu: the B200 drop-in module, loaded and called the way Memgraph does (through the fake mgp
-host), against the oracle, the committed e2e fixtures and -- where it was built -- the reference's
-own module loaded through the very same host."""
+host), against the oracle, the committed e2e fixtures and the committed rows of the reference's own
+module loaded through the very same host."""
 import json
 import os
 import threading
@@ -10,7 +10,8 @@ import pytest
 
 import _fakehost as fh
 from _checkers import Oracle
-from test_module_host import (HAVE_REF_MODULE, oracle_through_module_semantics, run_e2e_fixture, scattered_graph)
+from test_module_host import (MODULE_ARGS, module_rows_digests, oracle_through_module_semantics, run_e2e_fixture,
+                              scattered_graph)
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
@@ -58,13 +59,18 @@ def test_config1_graph_through_the_module(module, oracle, args):
     assert rel_err(ranks, exp) < REL_TOL
 
 
-@pytest.mark.skipif(not HAVE_REF_MODULE, reason="reference module not built")
-def test_same_rows_as_the_reference_module():
+def test_same_rows_as_the_reference_module(module, oracle):
+    """The reference module's rows on this graph are committed as digests (golden/pagerank_reference_module.json); the
+    oracle reproduces them bit for bit, so the B200 module is compared with the reference's rows through it."""
+    ref = json.load(open(os.path.join(GOLDEN, "pagerank_reference_module.json")))["same_rows"]
+    assert [c["args"] for c in ref] == [[], [20, 0.85, 0.0, 4], [7, 0.3, 0.0, 1]]
     gids, src, dst = scattered_graph(3000, 20000, seed=7)
-    with fh.Module(fh.MODULE_SO) as ours, fh.Module(fh.REF_MODULE_SO) as ref, fh.Graph(gids, src, dst) as g:
-        for args in [(), (20, 0.85, 0.0, 4), (7, 0.3, 0.0, 1)]:
-            n1, r1 = ours.call(g, *args)
-            n2, r2 = ref.call(g, *args)
+    with fh.Graph(gids, src, dst) as g:
+        for case in ref:
+            args = case["args"]
+            n2, r2, _ = oracle_through_module_semantics(oracle, gids, src, dst, **dict(zip(MODULE_ARGS, args)))
+            assert module_rows_digests(oracle, gids, src, dst, args) == case
+            n1, r1 = module.call(g, *args)
             assert np.array_equal(n1, n2)
             assert rel_err(r1, r2) < REL_TOL
 

@@ -1,14 +1,15 @@
 """Groundwork for the next path (Katz centrality, SURVEY 8f-1): oracle/katz_oracle.cpp pinned bit-exact against the
-reference's own katz.cpp compiled in place (oracle/_ref/libkatz_ref.so).  No GPU code exists for this path yet."""
+reference's own katz.cpp compiled in place (oracle/_ref/libkatz_ref.so), whose outputs are committed under golden/."""
 import ctypes
+import json
 import os
 
 import numpy as np
-import pytest
 
-from _checkers import ORACLE_SO, build_checkers
+from _checkers import ORACLE_SO, build_checkers, sha256_of
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 KATZ_REF_SO = os.path.join(REPO, "oracle", "_ref", "libkatz_ref.so")
 
 
@@ -49,17 +50,25 @@ def test_closed_form_on_a_chain():
     assert rc == 0 and it == 0 and not c.any()
 
 
-@pytest.mark.skipif(not os.path.exists(KATZ_REF_SO), reason="oracle/_ref/libkatz_ref.so not built (no reference checkout)")
-def test_bit_exact_vs_the_reference_katz():
+def katz_cases():
+    """The seeded graphs compared with the reference: yields (n, m, f, t, alpha, eps)."""
     rng = np.random.default_rng(17)
-    checked = 0
     for n, m in [(6, 9), (20, 40), (100, 250), (400, 1200), (1500, 3000)]:
         for alpha, eps in [(0.2, 1e-2), (0.05, 1e-3), (0.1, 1e-2)]:
             f, t = rng.integers(0, n, m), rng.integers(0, n, m)
-            rc, c, it = oracle_katz(n, f, t, alpha, eps, guard=2000)
-            if rc != 0:
-                continue  # does not separate within the guard (alpha^2 * deg_max >= 1): the reference would spin too
-            ref = ref_katz(n, f, t, alpha, eps)
-            assert np.array_equal(c, ref), (n, m, alpha, eps, it)
-            checked += 1
-    assert checked >= 8
+            yield n, m, f, t, alpha, eps
+
+
+def test_bit_exact_vs_the_reference_katz():
+    """The reference's centralities (tests/golden/katz_ref_outputs.json, written by make_golden.py from the reference's
+    own katz.cpp) are stored as the SHA-256 of their float64 bytes, so equality stays bit-exact."""
+    spec = json.load(open(os.path.join(GOLDEN, "katz_ref_outputs.json")))
+    expected = {(c["n"], c["m"], c["alpha"], c["eps"]): c["sha256"] for c in spec["cases"]}
+    checked = set()
+    for n, m, f, t, alpha, eps in katz_cases():
+        rc, c, it = oracle_katz(n, f, t, alpha, eps, guard=2000)
+        if rc != 0:
+            continue  # does not separate within the guard (alpha^2 * deg_max >= 1): the reference would spin too
+        assert sha256_of(c) == expected[(n, m, alpha, eps)], (n, m, alpha, eps, it)
+        checked.add((n, m, alpha, eps))
+    assert checked == set(expected) and len(checked) >= 8

@@ -1,21 +1,21 @@
-"""No-GPU tests of the drop-in boundary: the fake mgp host is validated by loading the REFERENCE's own
-pagerank module (BASELINE config #1), then the B200 module is checked for everything that does not
-need a device: exports, registered signature, argument validation, error texts, loud failure
-without a GPU, no leaked host objects."""
+"""No-GPU tests of the drop-in boundary: what the REFERENCE's own pagerank module returned through the
+fake mgp host (BASELINE config #1, committed under golden/) pins the oracle's module semantics, then
+the B200 module is checked for everything that does not need a device: exports, registered
+signature, argument validation, error texts, loud failure without a GPU, no leaked host objects."""
 import json
 import os
+import re
 import subprocess
 
 import numpy as np
 import pytest
 
 import _fakehost as fh
-from _checkers import Oracle
+from _checkers import Oracle, sha256_of
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HAVE_REF_MODULE = os.path.exists(fh.REF_MODULE_SO)
-needs_ref_module = pytest.mark.skipif(not HAVE_REF_MODULE, reason="oracle/_ref/pagerank_reference.so not built")
+MODULE_ARGS = ["max_iterations", "damping_factor", "stop_epsilon", "num_of_threads"]
 
 EXPECTED_SIGNATURE = ("get(max_iterations = 100 :: INTEGER, damping_factor = 0.84999999999999998 :: FLOAT, "
                       "stop_epsilon = 1.0000000000000001e-05 :: FLOAT, num_of_threads = 1 :: INTEGER) :: "
@@ -29,9 +29,9 @@ def oracle():
 
 @pytest.fixture(scope="module")
 def ref_module():
-    m = fh.Module(fh.REF_MODULE_SO)
-    yield m
-    m.close()
+    """What the reference's pagerank.so (oracle/_ref/pagerank_reference.so) did when loaded and called through this
+    host: tests/golden/pagerank_reference_module.json, written by make_golden.py."""
+    return json.load(open(os.path.join(GOLDEN, "pagerank_reference_module.json")))
 
 
 @pytest.fixture(scope="module")
@@ -60,67 +60,79 @@ def oracle_through_module_semantics(oracle, gids, src, dst, **kw):
     return order, ranks, it
 
 
-# ---- the host itself, validated with the reference's own module (config #1) ---------------------------------
+# ---- the reference's own module through this host (config #1), pinning the oracle's module semantics --------
 
-@needs_ref_module
 def test_reference_module_signature(ref_module):
-    assert ref_module.signature() == EXPECTED_SIGNATURE
+    assert ref_module["signature"] == EXPECTED_SIGNATURE
 
 
-@needs_ref_module
+def module_rows_digests(oracle, gids, src, dst, args):
+    """(nodes, ranks) the oracle says pagerank.get(*args) returns, as the digests the golden file stores."""
+    order, exp, _ = oracle_through_module_semantics(oracle, gids, src, dst, **dict(zip(MODULE_ARGS, args)))
+    return {"args": list(args), "nodes_sha256": sha256_of(order, np.int64), "ranks_sha256": sha256_of(exp)}
+
+
 def test_config1_reference_module_erdos_renyi_10k_50k(ref_module, oracle):
     """BASELINE config #1: 10k-node / 50k-edge Erdos-Renyi graph through the reference algorithm and
-    the C-ABI module loader, no GPU.  Default args and (20, 0.85, 0.0, 8)."""
-    n, m = 10_000, 50_000
-    gids, src, dst = scattered_graph(n, m, seed=42)
-    before = fh.live_objects()
-    with fh.Graph(gids, src, dst) as g:
-        nodes, ranks = ref_module.call(g)
-        nodes2, ranks2 = ref_module.call(g, 20, 0.85, 0.0, 8)
-    assert fh.live_objects() == before  # the reference module leaks nothing through this host
-    order, exp, _ = oracle_through_module_semantics(oracle, gids, src, dst)
-    assert np.array_equal(nodes, order)
-    assert np.array_equal(ranks, exp)  # same algorithm, same order of operations, T = 1
-    _, exp2, _ = oracle_through_module_semantics(oracle, gids, src, dst, max_iterations=20, stop_epsilon=0.0,
-                                                 num_of_threads=8)
-    assert np.array_equal(nodes2, order) and np.array_equal(ranks2, exp2)
+    the C-ABI module loader, no GPU.  Default args and (20, 0.85, 0.0, 8).  Same algorithm, same order
+    of operations, so the reference module's rows and the oracle's agree bit for bit."""
+    gids, src, dst = scattered_graph(10_000, 50_000, seed=42)
+    assert [c["args"] for c in ref_module["config1"]] == [[], [20, 0.85, 0.0, 8]]
+    for case in ref_module["config1"]:
+        assert module_rows_digests(oracle, gids, src, dst, case["args"]) == case
+
+
+def e2e_fixture_graph(case):
+    """(gid_of, gids, src, dst) of an e2e fixture: gids follow creation order."""
+    ids = sorted({v for e in case["edges_by_node_id"] for v in e})
+    gid_of = {node_id: 1000 + 3 * i for i, node_id in enumerate(ids)}
+    src = [gid_of[a] for a, _ in case["edges_by_node_id"]]
+    dst = [gid_of[b] for _, b in case["edges_by_node_id"]]
+    return gid_of, list(gid_of.values()), src, dst
+
+
+def e2e_fixture_rows(gid_of, nodes, ranks):
+    id_of = {v: k for k, v in gid_of.items()}
+    return sorted([id_of[int(gid)], float(r)] for gid, r in zip(nodes, ranks))  # ORDER BY node ASC
 
 
 def run_e2e_fixture(module, case):
-    ids = sorted({v for e in case["edges_by_node_id"] for v in e})
-    gid_of = {node_id: 1000 + 3 * i for i, node_id in enumerate(ids)}  # gids follow creation order here
-    src = [gid_of[a] for a, _ in case["edges_by_node_id"]]
-    dst = [gid_of[b] for _, b in case["edges_by_node_id"]]
-    with fh.Graph(list(gid_of.values()), src, dst) as g:
+    gid_of, gids, src, dst = e2e_fixture_graph(case)
+    with fh.Graph(gids, src, dst) as g:
         nodes, ranks = module.call(g, *case["call_args"])
-    id_of = {v: k for k, v in gid_of.items()}
-    rows = sorted((id_of[int(gid)], float(r)) for gid, r in zip(nodes, ranks))  # ORDER BY node ASC
-    return rows
+    return e2e_fixture_rows(gid_of, nodes, ranks)
 
 
-@needs_ref_module
-def test_reference_module_e2e_fixtures(ref_module):
-    """mage/tests/e2e/pagerank_test/*: expected rows at abs 1e-3 (test_module.py:21,76)."""
+def test_reference_module_e2e_fixtures(ref_module, oracle):
+    """mage/tests/e2e/pagerank_test/*: expected rows at abs 1e-3 (test_module.py:21,76); the oracle
+    returns exactly the reference module's rows."""
     spec = json.load(open(os.path.join(GOLDEN, "pagerank_e2e_cases.json")))
     assert {c["name"] for c in spec["cases"]} == {"test_chain", "test_empty", "test_influential_node",
-                                                  "test_influential_node_transfer"}
+                                                  "test_influential_node_transfer"} == set(ref_module["e2e"])
     for case in spec["cases"]:
-        rows = run_e2e_fixture(ref_module, case)
+        rows = ref_module["e2e"][case["name"]]
+        gid_of, gids, src, dst = e2e_fixture_graph(case)
+        order, ranks, _ = oracle_through_module_semantics(oracle, gids, src, dst,
+                                                          **dict(zip(MODULE_ARGS, case["call_args"])))
+        assert e2e_fixture_rows(gid_of, order, ranks) == rows, case["name"]
         assert len(rows) == len(case["output"])
         for (node, rank), exp in zip(rows, case["output"]):
             assert node == exp["node"] and abs(rank - exp["rank"]) < spec["tolerance_abs"], case["name"]
 
 
-@needs_ref_module
-def test_reference_module_unit_vectors_through_host(ref_module):
+def test_reference_module_unit_vectors_through_host(ref_module, oracle):
     spec = json.load(open(os.path.join(GOLDEN, "pagerank_unit_vectors.json")))
-    for case in spec["cases"]:
+    through_host = {c["case"]: c for c in ref_module["unit_vectors"]}
+    for i, case in enumerate(spec["cases"]):
         if case["m"] != len(case["edges"]):
+            assert i not in through_host
             continue
         gids = np.arange(case["n"], dtype=np.int64) * 5 + 11
         e = np.array(case["edges"], dtype=np.int64).reshape(-1, 2)
-        with fh.Graph(gids, gids[e[:, 0]] if len(e) else [], gids[e[:, 1]] if len(e) else []) as g:
-            nodes, ranks = ref_module.call(g)
+        nodes, ranks = np.array(through_host[i]["nodes"], dtype=np.int64), np.array(through_host[i]["ranks"])
+        order, exp_oracle, _ = oracle_through_module_semantics(oracle, gids, gids[e[:, 0]] if len(e) else [],
+                                                               gids[e[:, 1]] if len(e) else [])
+        assert np.array_equal(order, nodes) and np.array_equal(exp_oracle, ranks)
         assert np.array_equal(nodes, gids)
         exp = np.array(case["expected"])
         if len(exp):
@@ -128,20 +140,24 @@ def test_reference_module_unit_vectors_through_host(ref_module):
             assert err.max() < 1e-3 and err.mean() < 1e-3
 
 
-@needs_ref_module
-def test_host_argument_validation(ref_module):
+def test_host_argument_validation(ref_module, b200_module):
+    """The host rejects malformed calls before the procedure runs; the thread-count error is the
+    reference module's text under the calling module's name."""
     with fh.Graph([1, 2], [1], [2]) as g:
         with pytest.raises(fh.ProcedureError, match="must be of type FLOAT"):
-            ref_module.call(g, 10, 1)  # integer literal for damping_factor is rejected (cypher_types.hpp:95,104)
+            b200_module.call(g, 10, 1)  # integer literal for damping_factor is rejected (cypher_types.hpp:95,104)
         with pytest.raises(fh.ProcedureError, match="requires between 0 and 4 arguments"):
-            ref_module.call(g, 10, 0.85, 1e-5, 1, 7)
-        with pytest.raises(fh.ProcedureError, match=r"pagerank_reference\.get: Number of threads can't be zero \(0\)!"):
-            ref_module.call(g, 10, 0.85, 1e-5, 0)
+            b200_module.call(g, 10, 0.85, 1e-5, 1, 7)
+        with pytest.raises(fh.ProcedureError) as err:
+            b200_module.call(g, 10, 0.85, 1e-5, 0)
+    reference_text = ref_module["zero_threads_error"]
+    assert reference_text == "pagerank_reference.get: Number of threads can't be zero (0)!"
+    assert str(err.value) == "pagerank.get: " + reference_text.split(": ", 1)[1]
 
 
 # ---- the B200 module: everything that needs no device -------------------------------------------------------
 
-def test_b200_module_exports_and_imports():
+def test_b200_module_exports_and_imports(ref_module):
     out = subprocess.run(["nm", "-D", "--defined-only", fh.MODULE_SO], capture_output=True, text=True, check=True).stdout
     assert " T mgp_init_module" in out and " T mgp_shutdown_module" in out
     und = subprocess.run(["nm", "-D", "--undefined-only", fh.MODULE_SO], capture_output=True, text=True, check=True).stdout
@@ -159,17 +175,11 @@ def test_b200_module_exports_and_imports():
     assert set(imported) - set(strong) <= {"mgp_must_abort", "mgp_result_reserve", "mgp_log"}
     # nothing CUDA-related is left undefined: the runtime is linked statically (dlopen RTLD_NOW | RTLD_LOCAL)
     assert "cuda" not in und.lower() and "nccl" not in und.lower()
-    if HAVE_REF_MODULE:
-        ref_und = subprocess.run(["nm", "-D", "--undefined-only", fh.REF_MODULE_SO], capture_output=True, text=True,
-                                 check=True).stdout
-        assert sorted(l.split()[-1] for l in ref_und.splitlines() if " U mgp_" in l) == reference_imports
+    assert ref_module["imports"] == reference_imports
 
 
-def test_b200_module_signature_is_the_reference_signature(b200_module):
-    assert b200_module.signature() == EXPECTED_SIGNATURE
-    if HAVE_REF_MODULE:
-        with fh.Module(fh.REF_MODULE_SO) as ref:
-            assert ref.signature() == b200_module.signature()
+def test_b200_module_signature_is_the_reference_signature(b200_module, ref_module):
+    assert b200_module.signature() == EXPECTED_SIGNATURE == ref_module["signature"]
 
 
 def test_b200_module_error_paths_without_device(b200_module):
@@ -204,29 +214,41 @@ def test_b200_module_polls_must_abort_during_ingest(b200_module):
         assert g.abort_polls() >= 1
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/include"), reason="reference checkout not present")
-def test_module_compiles_against_the_reference_header(tmp_path):
-    """include/mgp_abi.h restates a slice of include/mg_procedure.h; compiling the module against the
-    reference header instead proves every call the module makes matches the real prototypes."""
-    obj = tmp_path / "contract.o"
-    subprocess.run(["g++", "-std=c++20", "-fsyntax-only", "-DMGB200_USE_REFERENCE_MGP_HEADER",
-                    "-I", "/root/reference/include", "-I", os.path.join(REPO, "include"),
-                    os.path.join(REPO, "memgraph_b200", "csrc", "pagerank_module.cpp")], check=True)
-    # and the enum values / struct layout restated in mgp_abi.h agree with the reference header
-    probe = tmp_path / "probe.cpp"
-    probe.write_text("""
-#include <cstdio>
-#include <cstddef>
-#include HEADER
-int main() {
-  printf("%d %d %d %d %zu %zu\\n", (int)mgp_error::MGP_ERROR_NO_ERROR, (int)mgp_error::MGP_ERROR_OUT_OF_RANGE,
-         (int)mgp_error::MGP_ERROR_NOT_YET_IMPLEMENTED, (int)mgp_log_level::MGP_LOG_LEVEL_CRITICAL,
-         sizeof(mgp_vertex_id), offsetof(mgp_vertex_id, as_int));
-}
-""")
-    outs = []
-    for header, inc in [('"mgp_abi.h"', os.path.join(REPO, "include")), ('"mg_procedure.h"', "/root/reference/include")]:
-        exe = tmp_path / ("probe_" + str(len(outs)))
-        subprocess.run(["g++", "-std=c++20", f"-DHEADER={header}", "-I", inc, str(probe), "-o", str(exe)], check=True)
-        outs.append(subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout)
-    assert outs[0] == outs[1] == "0 4 13 5 8 0\n"
+MGP_ENUMS = {"MGP_ERROR_": "mgp_error", "MGP_LOG_LEVEL_": "mgp_log_level", "MGP_VALUE_TYPE_": "mgp_value_type"}
+
+
+def mgp_abi_probe(header, include_dir, workdir):
+    """Compiles and runs a probe that prints, for every function and enumerator include/mgp_abi.h declares, the
+    function's mangled C++ type (return and parameter types, typeid) and the enumerator's value, plus the layout of
+    mgp_vertex_id, all as seen through `header`.  Returns {name: value}."""
+    text = open(os.path.join(REPO, "include", "mgp_abi.h")).read()
+    text = text[text.index("#else"):]  # the restated declarations, not the branch that includes the reference header
+    functions = sorted(set(re.findall(r"\b(mgp_\w+)\(", text)))
+    enumerators = sorted(set(re.findall(r"\b(MGP_(?:ERROR|LOG_LEVEL|VALUE_TYPE)_\w+)", text)))
+    lines = [f'printf("%s %s\\n", "{f}", typeid({f}).name());' for f in functions]
+    for e in enumerators:
+        enum = next(v for k, v in MGP_ENUMS.items() if e.startswith(k))
+        lines.append(f'printf("%s %d\\n", "{e}", (int){enum}::{e});')
+    lines.append('printf("sizeof(mgp_vertex_id) %zu\\n", sizeof(mgp_vertex_id));')
+    lines.append('printf("offsetof(mgp_vertex_id,as_int) %zu\\n", offsetof(mgp_vertex_id, as_int));')
+    probe = os.path.join(workdir, "mgp_abi_probe.cpp")
+    with open(probe, "w") as f:
+        f.write("#include <cstddef>\n#include <cstdio>\n#include <typeinfo>\n#include \"%s\"\nint main() {\n%s\n}\n"
+                % (header, "\n".join(lines)))
+    exe = os.path.join(workdir, "mgp_abi_probe")
+    subprocess.run(["g++", "-std=c++20", "-I", include_dir, probe, "-o", exe], check=True)
+    out = subprocess.run([exe], capture_output=True, text=True, check=True).stdout
+    return dict(line.split(" ", 1) for line in out.splitlines())
+
+
+def test_mgp_abi_matches_the_reference_header(tmp_path):
+    """include/mgp_abi.h restates a slice of the reference's include/mg_procedure.h.  Every prototype, enumerator and
+    the vertex-id layout it declares, probed through mgp_abi.h, equals what the same probe printed through the
+    reference header (tests/golden/mgp_abi_reference.json, written by make_golden.py), so every call the modules
+    make has the real prototype."""
+    ref = json.load(open(os.path.join(GOLDEN, "mgp_abi_reference.json")))["probe"]
+    ours = mgp_abi_probe("mgp_abi.h", os.path.join(REPO, "include"), str(tmp_path))
+    assert ours == ref
+    assert [ours[k] for k in ("MGP_ERROR_NO_ERROR", "MGP_ERROR_OUT_OF_RANGE", "MGP_ERROR_NOT_YET_IMPLEMENTED",
+                              "MGP_LOG_LEVEL_CRITICAL", "sizeof(mgp_vertex_id)", "offsetof(mgp_vertex_id,as_int)")] == \
+        ["0", "4", "13", "5", "8", "0"]
