@@ -67,8 +67,10 @@ uint64_t build_chunk_edges(uint64_t fallback) {
 struct DeviceArrays final : EdgeSource {  // the whole COO is resident: chunks are views
   const uint32_t *from, *to;
   const double *weight;  // nullable
+  const double *outw;    // [n] out-weight sums by vertex (with weight)
   uint64_t last_first = 0;
-  DeviceArrays(uint64_t count, const uint32_t *f, const uint32_t *t, const double *w = nullptr) : from(f), to(t), weight(w) {
+  DeviceArrays(uint64_t count, const uint32_t *f, const uint32_t *t, const double *w = nullptr, const double *ow = nullptr)
+      : from(f), to(t), weight(w), outw(ow) {
     m = count;
     chunk_edges = build_chunk_edges(count);
   }
@@ -80,6 +82,7 @@ struct DeviceArrays final : EdgeSource {  // the whole COO is resident: chunks a
   }
   const double *weights() const override { return weight ? weight + last_first : nullptr; }
   bool weighted() const override { return weight != nullptr; }
+  const double *out_weights() const override { return outw; }
 };
 
 struct RmatStream final : EdgeSource {  // the synthetic workload, generated chunk by chunk: no COO is ever materialised
@@ -309,6 +312,15 @@ int mgb200_graph_create_host_weighted_u32(int device, uint64_t n, uint64_t m, co
   rc = check_device(device);
   if (rc) return rc;
   MGB_CUDA(cudaSetDevice(device));
+  // out-weight sums, left to right in input edge order (cuGraph's out_w of every vertex): one fixed order, so the
+  // sums -- and every rank divided by them -- do not depend on the build's chunking or on thread timing
+  std::vector<double> outw;
+  try {
+    outw.assign(n, 0.0);
+  } catch (const std::bad_alloc &) {
+    set_error("out of host memory");
+    return MGB200_ERR_INVALID_ARGUMENT;
+  }
   for (uint64_t e = 0; e < m; ++e) {
     if (from[e] >= n || to[e] >= n) {
       set_error("edge endpoint out of range (>= number_of_nodes)");
@@ -318,21 +330,25 @@ int mgb200_graph_create_host_weighted_u32(int device, uint64_t n, uint64_t m, co
       set_error("edge weights must be non-negative numbers");
       return MGB200_ERR_INVALID_ARGUMENT;
     }
+    outw[from[e]] += weight[e];
   }
   uint32_t *d_from = nullptr, *d_to = nullptr;
-  double *d_w = nullptr;
+  double *d_w = nullptr, *d_outw = nullptr;
   auto cleanup = [&]() {
     cudaFree(d_from);
     cudaFree(d_to);
     cudaFree(d_w);
+    cudaFree(d_outw);
   };
   cudaError_t e;
   const uint64_t cnt = std::max<uint64_t>(m, 1);
   if ((e = cudaMalloc(&d_from, cnt * 4)) != cudaSuccess || (e = cudaMalloc(&d_to, cnt * 4)) != cudaSuccess ||
       (e = cudaMalloc(&d_w, cnt * 8)) != cudaSuccess ||
+      (e = cudaMalloc(&d_outw, std::max<uint64_t>(n, 1) * 8)) != cudaSuccess ||
       (e = cudaMemcpy(d_from, from, m * 4, cudaMemcpyHostToDevice)) != cudaSuccess ||
       (e = cudaMemcpy(d_to, to, m * 4, cudaMemcpyHostToDevice)) != cudaSuccess ||
-      (e = cudaMemcpy(d_w, weight, m * 8, cudaMemcpyHostToDevice)) != cudaSuccess) {
+      (e = cudaMemcpy(d_w, weight, m * 8, cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (e = cudaMemcpy(d_outw, outw.data(), n * 8, cudaMemcpyHostToDevice)) != cudaSuccess) {
     cleanup();
     return cuda_fail(e, "weighted COO upload", __FILE__, __LINE__);
   }
@@ -348,7 +364,7 @@ int mgb200_graph_create_host_weighted_u32(int device, uint64_t n, uint64_t m, co
   h->g.part_rank = 0;
   h->g.part_world = 1;
   {
-    DeviceArrays source(m, d_from, d_to, d_w);
+    DeviceArrays source(m, d_from, d_to, d_w, d_outw);
     rc = build_graph(h->g, source);
   }
   cleanup();

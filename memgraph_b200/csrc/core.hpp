@@ -176,7 +176,7 @@ struct Graph {
   double *heavy_sums = nullptr;   // [n_heavy] per-row gathered sums of the current iteration
   // optional edge weights (cuGraph-semantics variants only; one partition): parallel to heavy_idx / sell_idx, pad = 0
   double *heavy_w = nullptr, *sell_w = nullptr;
-  double *outw_l = nullptr;       // [n] sum of the out-edge weights by label (FP64 atomics: not bit-reproducible)
+  double *outw_l = nullptr;       // [n] sum of the out-edge weights by label (EdgeSource::out_weights, input order)
 
   // SELL class
   uint64_t n_slices = 0;
@@ -299,6 +299,9 @@ struct EdgeSource {
   // optional edge weights of the chunk last returned by get() (nullptr: unweighted graph)
   virtual const double *weights() const { return nullptr; }
   virtual bool weighted() const { return false; }
+  // weighted graphs: device array [n] by original vertex id, each vertex's out-edge weights summed left to right in
+  // input edge order -- the producer has seen every edge already, and one fixed order makes the sums reproducible
+  virtual const double *out_weights() const { return nullptr; }
 };
 
 // graph_build.cu

@@ -89,10 +89,10 @@ __global__ void edge_key_all_kernel(uint64_t m, const uint32_t *from, const uint
     key[e] = (static_cast<uint64_t>(label_of[to[e]]) << 32) | label_of[from[e]];
 }
 
-__global__ void out_weight_kernel(uint64_t m, const uint32_t *from, const double *w, const uint32_t *label_of, double *outw_l) {
+__global__ void out_weight_kernel(uint64_t n, const double *outw, const uint32_t *label_of, double *outw_l) {
   const uint64_t stride = static_cast<uint64_t>(gridDim.x) * blockDim.x;
-  for (uint64_t e = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; e < m; e += stride)
-    atomicAdd(outw_l + label_of[from[e]], w[e]);
+  for (uint64_t v = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; v < n; v += stride)
+    outw_l[label_of[v]] = outw[v];
 }
 
 __global__ void edge_key_owned_kernel(uint64_t m, const uint32_t *from, const uint32_t *to, const uint32_t *label_of,
@@ -653,10 +653,14 @@ int build_graph(Graph &g, EdgeSource &edges) {
   }
   double *eval = nullptr, *eval_alt = nullptr;  // weights travelling with the edge keys through the sort
   if (weighted) {
+    if (!edges.out_weights()) {
+      set_error("internal: a weighted edge source must supply its out-weight sums");
+      return MGB200_ERR_INVALID_ARGUMENT;
+    }
     MGB_CUDA(tmp.alloc(&eval, g.local_edges));
     MGB_CUDA(tmp.alloc(&eval_alt, g.local_edges));
     MGB_CUDA(keep_alloc(g, &g.outw_l, n));
-    MGB_CUDA(cudaMemsetAsync(g.outw_l, 0, n * sizeof(double), st));
+    out_weight_kernel<<<blocks_for(n, g.sm_count), kThreads, 0, st>>>(n, edges.out_weights(), g.label_of, g.outw_l);
   }
   if (m && g.part_world > 1) MGB_CUDA(cudaMemsetAsync(counts + 3, 0, sizeof(unsigned long long), st));
   for (uint64_t first = 0; first < m; first += chunk_cap) {  // pass 2 over the edge list: who reads what, owned edges
@@ -668,11 +672,8 @@ int build_graph(Graph &g, EdgeSource &edges) {
       need_mask_kernel<<<blocks_for(cnt, g.sm_count), kThreads, 0, st>>>(cnt, d_from, d_to, g.label_of, map, g.need_mask);
     if (g.part_world == 1) {
       edge_key_all_kernel<<<blocks_for(cnt, g.sm_count), kThreads, 0, st>>>(cnt, d_from, d_to, g.label_of, ekey + first);
-      if (weighted) {
-        const double *d_w = edges.weights();
-        MGB_CUDA(cudaMemcpyAsync(eval + first, d_w, cnt * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        out_weight_kernel<<<blocks_for(cnt, g.sm_count), kThreads, 0, st>>>(cnt, d_from, d_w, g.label_of, g.outw_l);
-      }
+      if (weighted)
+        MGB_CUDA(cudaMemcpyAsync(eval + first, edges.weights(), cnt * sizeof(double), cudaMemcpyDeviceToDevice, st));
     } else {
       edge_key_owned_kernel<<<blocks_for(cnt, g.sm_count), kThreads, 0, st>>>(cnt, d_from, d_to, g.label_of, map, row_hi,
                                                                              ekey, counts + 3);

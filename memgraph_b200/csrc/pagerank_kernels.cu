@@ -526,10 +526,11 @@ __global__ void __launch_bounds__(kBlockThreads, MGB_SELL_MIN_BLOCKS) sell_rows_
   sell_walk<kPath, false>(a, nullptr);
 }
 
-// every gathered value multiplied by its edge weight (cuGraph-semantics variants, one partition)
+// every gathered value multiplied by its edge weight (cuGraph-semantics variants, one partition); no hot table
+template <int kPath>
 __global__ void __launch_bounds__(kBlockThreads, MGB_SELL_MIN_BLOCKS) sell_rows_weighted_kernel(const SellArgs a) {
   if (ld_volatile_int(&a.state->done)) return;
-  sell_walk<kPathRange, false, true>(a, nullptr);
+  sell_walk<kPath, false, true>(a, nullptr);
 }
 
 // The same walk with the hot table: ONE 1024-thread CTA per SM (the same 32 warps as 4 x 256 threads) so that the SM
@@ -935,14 +936,12 @@ double zero_row_rank(const Graph &g, const IterateConfig &cfg) {
 int launch_sell_rows(Graph &g, const SellArgs &s) {
   const uint32_t table_n = s.window.table_n;
   if (s.w != nullptr) {
-    if (s.window.path != kPathRange) {
-      set_error("internal: weighted gathers exist for the single-partition range path only");
-      return MGB200_ERR_INVALID_ARGUMENT;
-    }
-    const int grid = static_cast<int>(std::min(
-        static_cast<uint64_t>(grid_for(g, reinterpret_cast<const void *>(sell_rows_weighted_kernel))),
-        ceil_div(g.sell_work, kWarpsPerBlock)));
-    sell_rows_weighted_kernel<<<grid, kBlockThreads, 0, g.stream>>>(s);
+    void (*const fn)(SellArgs) = s.window.path == kPathFlags    ? sell_rows_weighted_kernel<kPathFlags>
+                                 : s.window.path == kPathLookup ? sell_rows_weighted_kernel<kPathLookup>
+                                                                : sell_rows_weighted_kernel<kPathRange>;
+    const int grid = static_cast<int>(std::min(static_cast<uint64_t>(grid_for(g, reinterpret_cast<const void *>(fn))),
+                                               ceil_div(g.sell_work, kWarpsPerBlock)));
+    fn<<<grid, kBlockThreads, 0, g.stream>>>(s);
   } else if (table_n > 0 && s.window.path != kPathLookup) {
     void (*const fn)(SellArgs) = s.window.path == kPathFlags ? sell_rows_table_kernel<kPathFlags> : sell_rows_table_kernel<kPathRange>;
     const int bytes = static_cast<int>(table_n * sizeof(double));
@@ -1143,8 +1142,9 @@ int launch_iteration(Graph &g, uint64_t it, const IterateConfig &cfg, uint64_t *
 int launch_gather_phase(Graph &g, const double *vec_in, uint64_t *launch_count, bool heavy_row_sums, bool weighted) {
   uint64_t launches = 0;
   const GatherWindow window = make_window(g);
-  if (weighted && (window.path != kPathRange || (g.n_slices > 0 && !g.sell_w) || (g.n_seg > 0 && !g.heavy_w))) {
-    set_error("this graph handle carries no edge weights (or is partitioned)");
+  // (partitioned handles never carry weights: build_graph refuses them)
+  if (weighted && ((g.n_slices > 0 && !g.sell_w) || (g.n_seg > 0 && !g.heavy_w))) {
+    set_error("this graph handle carries no edge weights");
     return MGB200_ERR_INVALID_ARGUMENT;
   }
   if (g.n_slices > 0) {
@@ -1181,10 +1181,13 @@ int launch_gather_phase(Graph &g, const double *vec_in, uint64_t *launch_count, 
     h.contrib_in = vec_in;
     h.window = window;
     h.state = g.state;
-    void (*const heavy_fn)(HeavyArgs) = (weighted && g.heavy_w)          ? heavy_segments_kernel<kPathRange, true>
-                                        : window.path == kPathFlags    ? heavy_segments_kernel<kPathFlags>
-                                        : window.path == kPathLookup ? heavy_segments_kernel<kPathLookup>
-                                                                     : heavy_segments_kernel<kPathRange>;
+    void (*const heavy_fn)(HeavyArgs) =
+        weighted ? (window.path == kPathFlags    ? heavy_segments_kernel<kPathFlags, true>
+                    : window.path == kPathLookup ? heavy_segments_kernel<kPathLookup, true>
+                                                 : heavy_segments_kernel<kPathRange, true>)
+                 : (window.path == kPathFlags    ? heavy_segments_kernel<kPathFlags>
+                    : window.path == kPathLookup ? heavy_segments_kernel<kPathLookup>
+                                                 : heavy_segments_kernel<kPathRange>);
     const int grid = static_cast<int>(std::min(static_cast<uint64_t>(grid_for(g, reinterpret_cast<const void *>(heavy_fn))),
                                                ceil_div(g.n_seg, kWarpsPerBlock)));
     heavy_fn<<<grid, kBlockThreads, 0, g.stream>>>(h);

@@ -4,8 +4,11 @@
 // policies); only the vector preparation (contribution + dangling mass) and the row epilogue differ:
 //   prepare : contrib[l] = pr[l] / outdeg[l] (0 for sinks), dangling = sum of pr over sinks      one pass over N labels
 //   epilogue: new[r] = alpha * gathered[r] + (alpha * dangling + 1 - alpha) * p[r], L1 diff       one pass over N rows
-// Both reductions are two-stage with a fixed tree (per-block partials, then one block): bit-reproducible run to run,
-// which cuGraph itself is not.  One partition: label == local row, so pr, p and the gathered sums share one index space.
+// Both reductions are two-stage with a fixed tree (per-block partials, then one block), every row is gathered in a
+// fixed order, and the out-weight sums of a weighted handle are summed on the host in input edge order
+// (mgb200_graph_create_host_weighted_u32): results are bit-reproducible run to run and handle to handle, whatever the
+// gather configuration or build chunking, which cuGraph itself is not.  One partition: label == local row, so pr, p and
+// the gathered sums share one index space.
 #include <algorithm>
 #include <vector>
 

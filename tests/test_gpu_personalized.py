@@ -81,7 +81,8 @@ def test_rmat_scale18_all_row_classes_and_errors():
 def test_edge_weights(seed, monkeypatch):
     """weight_property path: one non-negative FP64 weight per edge (mgb200_graph_create_host_weighted_u32); every gathered
     value is multiplied by its weight, contributions are divided by the out-WEIGHT sums.  Zero weights are legal (a vertex
-    whose out-edges all weigh 0 is dangling).  Tolerance: the out-weight sums are accumulated with FP64 atomics."""
+    whose out-edges all weigh 0 is dangling).  Tolerance: the out-weight sums equal the oracle's bit for bit (both add
+    in input edge order), but the device sums every row in source-label order, the oracle in edge order."""
     rng = np.random.default_rng(100 + seed)
     n = int(rng.integers(300, 4000))
     m = int(n * rng.integers(3, 10))
