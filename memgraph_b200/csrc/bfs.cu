@@ -8,10 +8,16 @@
 //   bottom-up  large frontiers: every unvisited vertex scans its REVERSE adjacency for a parent in the
 //              frontier bitmap (2 MiB at scale-24: L1/L2 resident) and stops at the first hit.
 // HBM-bound integer work: coalesced adjacency reads, random 4-byte depth / 1-bit frontier probes.
+//
+// MGB200_BFS_STRATEGY, read at every mgb200_bfs_run call, pins the strategy so that tests can reach every path on
+// small graphs: unset or "auto" = the switch above; "top_down" / "bottom_up" = that strategy at every level (bottom-up
+// from level 0, a one-vertex frontier); "alternate" = top-down on even levels, bottom-up on odd ones, so both hand-offs
+// between queue and bitmap run.  Any other value is refused, so that a typo cannot quietly run the default.
 #include <algorithm>
 #include <climits>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <cub/cub.cuh>
 #include <new>
 #include <vector>
@@ -264,6 +270,21 @@ int build_side(mgb200_bfs_graph &g, Scratch &tmp, const uint32_t *row, const uin
   return MGB200_OK;
 }
 
+enum class Strategy { kAuto, kTopDown, kBottomUp, kAlternate };
+
+int read_strategy(Strategy *out) {
+  const char *s = getenv("MGB200_BFS_STRATEGY");
+  if (!s || !strcmp(s, "auto")) *out = Strategy::kAuto;
+  else if (!strcmp(s, "top_down")) *out = Strategy::kTopDown;
+  else if (!strcmp(s, "bottom_up")) *out = Strategy::kBottomUp;
+  else if (!strcmp(s, "alternate")) *out = Strategy::kAlternate;
+  else {
+    set_error(std::string("bfs: unknown MGB200_BFS_STRATEGY '") + s + "' (auto, top_down, bottom_up or alternate)");
+    return MGB200_ERR_INVALID_ARGUMENT;
+  }
+  return MGB200_OK;
+}
+
 int read_counters(mgb200_bfs_graph &g) {
   MGB_CUDA(cudaMemcpyAsync(g.host_counters, g.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, g.stream));
   MGB_CUDA(cudaStreamSynchronize(g.stream));
@@ -419,6 +440,8 @@ int mgb200_bfs_run(mgb200_bfs_graph *g, uint64_t source, int direction, int64_t 
     set_error("bfs: source vertex out of range");
     return MGB200_ERR_INVALID_ARGUMENT;
   }
+  Strategy strategy = Strategy::kAuto;
+  if (int rc = read_strategy(&strategy)) return rc;
   MGB_CUDA(cudaSetDevice(g->device));
   cudaStream_t st = g->stream;
   const uint64_t n = g->n;
@@ -457,7 +480,10 @@ int mgb200_bfs_run(mgb200_bfs_graph *g, uint64_t source, int direction, int64_t 
     explored_degree += m_f;
     stats.kernel_launches++;
     // Beamer's switch: go bottom-up when the frontier's edges outnumber 1/14 of the unexplored ones
-    const bool bottom_up = m_f > m_u / 14 && nf > 1024;
+    bool bottom_up = m_f > m_u / 14 && nf > 1024;
+    if (strategy == Strategy::kTopDown) bottom_up = false;
+    else if (strategy == Strategy::kBottomUp) bottom_up = true;
+    else if (strategy == Strategy::kAlternate) bottom_up = (level & 1) != 0;
     MGB_CUDA(cudaMemsetAsync(g->counters, 0, 2 * sizeof(unsigned long long), st));
     if (bottom_up) {
       clear_words_kernel<<<blocks_for(words, g->sm_count), kThreads, 0, st>>>(words, g->bitmap[0]);
